@@ -1,6 +1,6 @@
 """bench.py — headline benchmark of the post-processing hot path (driver contract: DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Headline workload = the configuration BASELINE.json's metric is quoted on ("grain+LUT+colormatch+sharpen chain at 4K"), i.e. the
@@ -16,8 +16,8 @@ One "step" = one pass of the chain over the rank's frames:
           H2D and D2H copies inside the timed region; e2e.stock_nodes = the same chain as four unchanged ComfyUI nodes
   extra : configs[1] (64 x 1080p fp16, grain + LUT + unsharp), "grain + LUT + unsharp at 4K fp32", configs[2] (colour match alone: LAB
           transfer and histogram mode, reference statistics gathered every step), configs[4] (temporal sharpen), each with its own roofline
-  --impl reference : the reference's CPU path for the same chain (oracle port of the reference nodes; /root/reference
-          does not exist on the GPU box) on all host cores, rank 0 only, bounded sample per step
+  --impl reference : the reference's CPU path for the same chain (oracle port of the reference nodes, so the reference's own
+          source is not needed) on all host cores, rank 0 only, 2 frames per step, --steps timed steps
 """
 import argparse
 import importlib
@@ -150,6 +150,22 @@ def device_natural_frames(n, h, w, seed, dtype, dev):
     return (acc * gain + off).clamp_(0, 1).permute(0, 2, 3, 1).contiguous().to(dtype)
 
 
+DUMP_PIXELS = 1 << 21          # sampled output pixels over all ranks: 2 Mi x 3 channels x 4 B = 24 MiB
+DUMP_CROP = 256                # side of the full-resolution corner crops (the stencil's replicated border is in them)
+
+
+def headline_outputs(out, ref_sums, rank, world):
+    """What the last headline step returned, small enough to store: a fixed, seeded sample of the output pixels (the same
+    positions on every run and every build), full-resolution corner crops of the rank's first and last frame, and the
+    gathered reference statistics.  float32 / float64 host arrays keyed by file name."""
+    B, H, W, C = out.shape
+    g = torch.Generator().manual_seed(7 + rank)
+    idx = torch.randint(0, B * H * W, (max(1, DUMP_PIXELS // world),), generator=g).sort().values
+    arrays = {"pixels": out.view(-1, C)[idx.to(out.device)], "first_frame_top_left": out[0, :DUMP_CROP, :DUMP_CROP],
+              "last_frame_bottom_right": out[-1, -DUMP_CROP:, -DUMP_CROP:], "ref_sums": ref_sums}
+    return {"rank%d_%s" % (rank, k): v.cpu().numpy() for k, v in arrays.items()}
+
+
 def tile_frames(base, total):
     """`total` frames from the distinct `base` frames (repeated; a per-frame offset keeps every frame's statistics distinct)"""
     n = base.shape[0]
@@ -202,7 +218,7 @@ def run_reference(args):
         c = oracle.apply_lut(b, lut, 10.0)
         return oracle.unsharp_numpy(c, SHARPEN)
     step()
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
         step()
@@ -290,6 +306,8 @@ def run_b200(args):
     sampler.start()
     ms_step, launches = timed(step, args.steps, 0)
     sampler.stop_flag.set()
+    # taken before the schedules and extra lines below overwrite `out`
+    dump = headline_outputs(out, chain._ref_sums, rank, world) if args.dump_outputs else None
     value = world * npix / 1e6 / (ms_step / 1e3)
     tile_path = nv.last_tile_path()
     ref_sums_identical = True
@@ -487,6 +505,11 @@ def run_b200(args):
                                     "sample": "1 x 3840x2160 fp32 frame, best of 2, oracle port of FastFilmGrain -> ColorMatchToReference -> VRGDG_LUTS -> "
                                               "FastUnsharpSharpen (%.1f s)" % secs}
         print(json.dumps(line))
+    if dump is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if dist is not None:
         dist.destroy_process_group()
 
@@ -499,7 +522,13 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra lines and the stock-node leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps write a fixed sample of the last headline step's outputs "
+                                                          "to DIR/<name>.npy (float32 / float64, under 40 MB), to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs stores the B200 path's outputs; --impl reference has none to store")
     if args.impl == "reference":
         run_reference(args)
     else:

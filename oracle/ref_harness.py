@@ -1,8 +1,9 @@
-"""Executes the REFERENCE's own source for the hot path — TEST INFRASTRUCTURE, container-only.
+"""Executes the REFERENCE's own source for the hot path — TEST INFRASTRUCTURE.
 
-/root/reference exists only in the build container (never on the GPU box), so nothing under `-m gpu`,
-smoke() or bench.py may import this module.  It is used by tests/golden/make_golden.py to freeze golden
-vectors and by tests/test_oracle_golden.py (skipped when the tree is absent) to pin oracle/vrgdg_oracle.py.
+The reference (the original comfyui-vrgamedevgirl node pack) is not part of this repository.  It is looked for where
+VRGDG_REFERENCE_ROOT points, else in the git-ignored oracle/_ref/, else at /root/reference, where the golden vectors were
+frozen from.  Nothing under `-m gpu`, smoke() or bench.py may import this module.  It is used by tests/golden/make_golden.py
+to freeze golden vectors and by tests/test_oracle_golden.py (skipped without a reference checkout) to pin oracle/vrgdg_oracle.py.
 
 Technique = the reference's own tests (tests/test_standalone_video_enhancer.py:19-36): ast.parse the file,
 keep the wanted top-level definitions, exec them in a namespace of stand-ins for what ComfyUI provides.
@@ -19,7 +20,16 @@ import numpy as np
 import torch
 import torch.nn.functional as F
 
-REFERENCE_ROOT = os.environ.get("VRGDG_REFERENCE_ROOT", "/root/reference")
+def _reference_root():
+    if os.environ.get("VRGDG_REFERENCE_ROOT"):
+        return os.environ["VRGDG_REFERENCE_ROOT"]
+    for root in (os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"), "/root/reference"):
+        if os.path.isfile(os.path.join(root, "nodes.py")):
+            return root
+    return "/root/reference"
+
+
+REFERENCE_ROOT = _reference_root()
 
 
 def available():

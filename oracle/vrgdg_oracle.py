@@ -7,8 +7,8 @@ Each function restates, with the same torch / numpy calls in the same order, wha
 computes (citations are file:line into the reference tree), so that on a CPU it produces bit-identical
 tensors.  Pinning: tests/golden/*.npz were produced by executing the reference's own source
 (oracle/ref_harness.py, AST-extracted exactly like the reference's tests do) and
-tests/test_oracle_golden.py checks this restatement against them; in a container that still has
-/root/reference the same test also compares against the live reference code.
+tests/test_oracle_golden.py checks this restatement against them; where a checkout of the reference is found
+(oracle/ref_harness.py: VRGDG_REFERENCE_ROOT) the same test also compares against the live reference code.
 
 Parity status
   * grain / unsharp / laplacian / sobel / 3D LUT / cube parser / palette LUT / u8 codecs: PINNED by the

@@ -1,7 +1,7 @@
 """Freezes golden input/output vectors by EXECUTING THE REFERENCE'S OWN SOURCE (oracle/ref_harness.py).
 
-Run in the build container only (needs /root/reference):   python tests/golden/make_golden.py
-The .npz / .json files it writes are committed; GPU-box tests read them and never touch /root/reference.
+Needs a checkout of the reference:   VRGDG_REFERENCE_ROOT=<checkout> python tests/golden/make_golden.py
+The .npz / .json files it writes are committed; the tests read them and never need the reference.
 """
 import hashlib
 import json
@@ -17,7 +17,7 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import ref_harness as RH  # noqa: E402
-from helpers import LUTS, natural_frames, white_frames  # noqa: E402
+from helpers import LUTS, natural_frames, save_golden, white_frames  # noqa: E402
 
 warnings.filterwarnings("ignore")
 torch.set_num_threads(4)
@@ -25,7 +25,7 @@ torch.set_num_threads(4)
 
 def save(name, **arrays):
     out = {k: (v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)) for k, v in arrays.items()}
-    np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
+    save_golden(name, out, HERE)
     print(name, {k: tuple(v.shape) for k, v in out.items()})
 
 

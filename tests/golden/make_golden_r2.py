@@ -1,6 +1,6 @@
 """Round-2 additions to the golden vectors, produced by EXECUTING THE REFERENCE'S OWN SOURCE (oracle/ref_harness.py).
 
-Run in the build container only (needs /root/reference):   python tests/golden/make_golden_r2.py
+Needs a checkout of the reference:   VRGDG_REFERENCE_ROOT=<checkout> python tests/golden/make_golden_r2.py
   lut_big.npz : VRGDG_LUTS._parse_cube_file + _apply_cube_lut + the strength blend of apply_lut on generated 64^3 / 65^3 tables
                 (tests/helpers.py::write_big_cube; the 65^3 file carries integer DOMAIN_MIN/MAX lines)
 """

@@ -1,5 +1,6 @@
 """Shared test helpers: synthetic frames and golden loading."""
 import os
+import re
 
 import numpy as np
 import torch
@@ -31,8 +32,35 @@ def natural_frames(B, H, W, seed=0, dtype=torch.float32, device="cpu"):
     return (acc + off).clamp(0, 1).permute(0, 2, 3, 1).contiguous().to(dtype).to(device)
 
 
-def load_golden(name):
-    return dict(np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False))
+GOLDEN_FILE_BYTES = 1000000      # no stored vector file is larger than this: save_golden spreads the arrays over more files
+
+
+def load_golden(name, directory=GOLDEN):
+    """The arrays of tests/golden/<name>.npz and of its continuation files <name>_part<k>.npz."""
+    out = {}
+    for f in sorted(os.listdir(directory)):
+        if f == name + ".npz" or re.fullmatch(re.escape(name) + r"_part\d+\.npz", f):
+            with np.load(os.path.join(directory, f), allow_pickle=False) as z:
+                out.update({k: z[k] for k in z.files})
+    return out
+
+
+def save_golden(name, arrays, directory=GOLDEN, limit=GOLDEN_FILE_BYTES):
+    """np.savez_compressed `arrays` as <name>.npz, spread round-robin over <name>_part2.npz, _part3.npz, ... when one file would be
+    larger than `limit` bytes.  load_golden(name) returns them as one dict again."""
+    keys = list(arrays)
+    for f in os.listdir(directory):
+        if re.fullmatch(re.escape(name) + r"_part\d+\.npz", f):
+            os.remove(os.path.join(directory, f))
+    for n in range(1, len(keys) + 1):
+        paths = [os.path.join(directory, name + (".npz" if i == 0 else "_part%d.npz" % (i + 1))) for i in range(n)]
+        for i, path in enumerate(paths):
+            np.savez_compressed(path, **{k: arrays[k] for k in keys[i::n]})
+        if all(os.path.getsize(p) <= limit for p in paths):
+            return paths
+        for path in paths[1:]:
+            os.remove(path)
+    raise ValueError("one array of %s is larger than %d bytes compressed" % (name, limit))
 
 
 def t(a):

@@ -1,5 +1,5 @@
 import importlib, os, sys, json, torch
-ROOT="/root/repo"
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 pkg = importlib.import_module("comfyui-vrgamedevgirl_b200")
 from helpers import LUTS, natural_frames
